@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Gbases/s of fastplong's per-read hot loop (adapter-trim + Q-filter + stats) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): 1M DISTINCT ONT-like reads, mean 15 kb (32 GB of payload, generated on the
 device), adapters as the reference's evaluator auto-detects them on this generator's reads, --cut_front --cut_tail
@@ -12,6 +12,9 @@ oracle, every word of both Stats blocks against an independent torch restatement
 One step = one pass of processSingleEnd over the whole per-GPU batch (+ the Stats/FilterResult all-reduce when N>1).
 `value` = device-resident throughput; `e2e` = the same metric through fpl_process_host with pinned HOST buffers
 (H2D of every byte + D2H of the per-read records inside the timed region).
+--dump-outputs DIR writes what the last timed step computed as DIR/<name>.npy (float64, exact): both Stats blocks, the
+FilterResult counters and the per-read records of a fixed, seeded sample of the reads.  The inputs depend on the arguments
+only, so two builds can be compared file by file.
 
 --impl reference times the reference's own CPU implementation (oracle/_ref/fastplong_ref, built from the
 unmodified sources) on a bounded sample of the same workload with all host threads it can use.
@@ -44,6 +47,8 @@ FULL_CHECK_BASES = 24_000_000   # ... this many bases in total
 FULL_CHECK_BUDGET_S = 150   # the torch restatement of the Stats blocks gives up beyond this (reported, not fatal)
 E2E_SUBMISSIONS = 64        # host submissions per step of the end-to-end leg
 E2E_HOST_CHUNKS = 4         # distinct pinned host chunks cycled through them
+DUMP_BYTES = 64 << 20       # --dump-outputs: at most this much in all
+DUMP_MAX_READS = 1 << 17    # ... and the records of at most this many reads
 
 
 # name: (reads per GPU, replicas, mean length, generator keywords, description)
@@ -241,6 +246,35 @@ def full_scale_check(torch, eng, opt, tile, d_seq, d_qual, offsets, lens, tile_r
     return out
 
 
+def dump_outputs(eng, n_reads, cycles, out_dir):
+    """What the caller of the timed path receives after a step: both Stats blocks (laid out over the longest read's
+    cycles), the counters and the per-read records, one .npy per field.  The records are those of a fixed, seeded sample
+    of the reads (sorted read indices in records_read_index.npy) sized so that everything stays within DUMP_BYTES; a Stats
+    block above 3/8 of DUMP_BYTES (reads of hundreds of kb) is cut to a fixed, seeded sample of its words the same way."""
+    from fastplong_b200.abi import RESULT_DTYPE
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"counters": eng.counters()}
+    for which, name in ((0, "stats_pre"), (1, "stats_post")):
+        block = eng.stats(which, cycles)
+        if block.size * 8 > DUMP_BYTES * 3 // 8:
+            arrays[name + "_index"] = np.sort(np.random.default_rng(SEED + which).choice(block.size, DUMP_BYTES // 64,
+                                                                                          replace=False))
+            block = block[arrays[name + "_index"]]
+        arrays[name] = block
+    fixed = sum(a.size for a in arrays.values()) * 8
+    per_read = 8 * (1 + sum(int(np.prod(RESULT_DTYPE[f].shape or (1,))) for f in RESULT_DTYPE.names))
+    k = int(min(n_reads, DUMP_MAX_READS, max(0, DUMP_BYTES - fixed) // per_read))
+    idx = np.sort(np.random.default_rng(SEED).choice(n_reads, size=k, replace=False)) if k < n_reads else np.arange(n_reads)
+    res = eng.fetch_results(n_reads)[idx]
+    arrays["records_read_index"] = idx
+    for f in RESULT_DTYPE.names:
+        arrays["records_" + f] = res[f]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    return {"dir": out_dir, "files": len(arrays), "sampled_reads": k,
+            "bytes": int(sum(np.asarray(a).size for a in arrays.values()) * 8)}
+
+
 def h2d_peak_gbs(torch, dev):
     """Pinned host -> device copy bandwidth of this box (the roofline of the end-to-end leg)."""
     n = 1 << 30
@@ -393,6 +427,7 @@ def run_ours(args):
     launches = eng.launch_count - l0
     ktimes = eng.kernel_times()
     eng.set_timing(False)
+    dumped = dump_outputs(eng, n_reads, int(tile.lens.max()), args.dump_outputs) if args.dump_outputs and rank == 0 else None
     if world > 1:
         # every rank's clocks and step time: the value is the max over ranks, so a GPU that ran slower (power cap under an
         # 8-GPU load) shows here
@@ -567,6 +602,8 @@ def run_ours(args):
         "collective_ms": kern.get("nccl_allreduce(stats)", {}).get("ms_per_step") if world > 1 else None,
         "roofline": roofline, "kernels": kern, "cpu_baseline": cpu_baseline,
     }
+    if dumped:
+        line["dumped_outputs"] = dumped
     emit(line)
 
 
@@ -705,7 +742,11 @@ def main():
     ap.add_argument("--no-full-check", action="store_true", help="profiling aid: skip the full-size parity check behind the timed legs")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="profiling aid: skip the end-to-end leg (keeps an ncu launch list short)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (Stats blocks, counters, sampled records)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -10,12 +10,17 @@ where /root/reference exists and oracle/_ref has been built by `make -C oracle`)
   binary_<name>.json             whole-binary runs of oracle/_ref/fastplong_ref on a seeded FASTQ: md5 of --out and
                                  --failed_out, md5 of the JSON report text minus its "command" line, the report's
                                  scalar sections (curves replaced by their md5), and the input md5
+  reference_outputs.json         what the reference computed in the tests that compare with it (tests/reference_outputs.py):
+                                 those tests are called here with the reference running in place of the stored outputs
 
-Usage:  python tests/golden/make_golden.py
+Usage:  python tests/golden/make_golden.py [reference_outputs]     (the argument: only reference_outputs.json)
 """
 import hashlib
+import inspect
+import itertools
 import json
 import os
+import pathlib
 import subprocess
 import sys
 import tempfile
@@ -114,5 +119,59 @@ def main():
     print("golden fixtures written to", HERE)
 
 
+# the tests that compare with the reference; the GPU ones stop once the reference has run (reference_outputs.Recorded)
+REFERENCE_TESTS = {
+    "test_oracle_vs_reference": None,
+    "test_evaluator": ["test_host_logic_matches_reference_binary"],
+    "test_gpu_binary": ["test_gpu_binary_matches_reference_binary", "test_gpu_binary_mask_break_matches_reference_binary",
+                        "test_config1_full_size_bit_exact", "test_gpu_binary_non_strict_fastq_like_reference",
+                        "test_gpu_binary_many_small_chunks", "test_gpu_binary_file_size_is_a_multiple_of_the_chunk",
+                        "test_gpu_binary_plus_lines_kept_verbatim"],
+    "test_gpu_multigpu": ["test_drop_in_binary_workers_over_two_gpus"],
+}
+
+
+def parameter_sets(fn):
+    """Every keyword set pytest would call `fn` with (its parametrize marks, crossed)."""
+    axes = []
+    for m in getattr(fn, "pytestmark", []):
+        if m.name != "parametrize":
+            continue
+        names = [n.strip() for n in m.args[0].split(",")] if isinstance(m.args[0], str) else list(m.args[0])
+        axes.append([dict(zip(names, v if len(names) > 1 else (v,))) for v in m.args[1]])
+    for combo in itertools.product(*axes):
+        yield {k: v for d in combo for k, v in d.items()}
+
+
+def record_reference_outputs():
+    import importlib
+    import reference_outputs
+    rec = reference_outputs.RECORDING = {}
+    for modname, names in REFERENCE_TESTS.items():
+        mod = importlib.import_module(modname)
+        if modname == "test_gpu_multigpu":
+            mod._n_gpus = lambda: 2              # only the reference half runs here
+        reference_outputs.STOP_AFTER_RECORD = modname.startswith("test_gpu")
+        for name in names or [n for n in dir(mod) if n.startswith("test_")]:
+            fn = getattr(mod, name)
+            for kw in parameter_sets(fn):
+                keys = set(rec)
+                with tempfile.TemporaryDirectory() as d:
+                    if "tmp_path" in inspect.signature(fn).parameters:
+                        kw["tmp_path"] = pathlib.Path(d)
+                    try:
+                        fn(**kw)
+                    except reference_outputs.Recorded:
+                        pass
+                assert set(rec) != keys or modname.startswith("test_gpu"), (name, kw)
+    reference_outputs.RECORDING = None
+    with open(reference_outputs.PATH, "w") as f:
+        json.dump(rec, f, indent=0, sort_keys=True)
+        f.write("\n")
+    print(len(rec), "reference outputs written to", reference_outputs.PATH)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] != ["reference_outputs"]:
+        main()
+    record_reference_outputs()

@@ -143,6 +143,17 @@ def build_library(override=None):
 _emu_bin_path = None
 
 
+def _reference_src():
+    """The reference's source directory, whose headers seprocessor_gpu.cpp includes: oracle/Makefile's REF (which the
+    environment may override), so that the emulated build and the Makefiles read the same sources."""
+    r = subprocess.run(["make", "-s", "--no-print-directory", "-C", os.path.join(ROOT, "oracle"), "print-ref"],
+                       capture_output=True, text=True)
+    return os.path.join(r.stdout.strip(), "src") if r.returncode == 0 and r.stdout.strip() else None
+
+
+REF_SRC = _reference_src()
+
+
 def build_binary():
     """-> path of fastplong_gpu_emu: host/seprocessor_gpu.cpp (unchanged) + the reference's unmodified objects (oracle/_ref/obj, as
     fastplong_b200/host/Makefile links them) + the emulated library.  The drop-in CLI without a GPU."""
@@ -163,8 +174,9 @@ def build_binary():
         san = os.environ.get("FPL_EMU_SANITIZE", "")
         sflags = [f"-fsanitize={san}", "-fno-omit-frame-pointer", "-g"] if san else []
         subprocess.check_call(["g++", "-std=c++14", "-pthread", "-O2", "-w", *sflags, "-I", os.path.join(SIMT, "fake"), "-I", os.path.join(ROOT, "oracle", "shim"),
-                               "-I", "/root/reference/src", "-I", os.path.join(ROOT, "include"), "-c", host, "-o", obj])
-        refobj = sorted(os.path.join(objdir, f) for f in os.listdir(objdir) if f.endswith(".o") and f != "seprocessor.o")
+                               "-I", REF_SRC, "-I", os.path.join(ROOT, "include"), "-c", host, "-o", obj])
+        refobj = sorted(os.path.join(objdir, f) for f in os.listdir(objdir)
+                        if f.endswith(".o") and f not in ("seprocessor.o", "seprocessor_gpu.o"))
         subprocess.check_call(["g++", "-pthread", *sflags[:1], "-o", exe, obj, *refobj, lib, "-lz", "-ldl", f"-Wl,-rpath,{out}"])
         open(stamp, "w").write(tag)
     _emu_bin_path = exe

@@ -62,8 +62,9 @@ def test_fastq_text_through_the_emulated_c_abi(emulated_binding):
     g.close()
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN) or not os.path.exists(os.path.join(simt_emu.ROOT, "oracle", "_ref", "obj", "main.o")),
-                    reason="oracle/_ref (the reference's objects and binary) not built")
+@pytest.mark.skipif(not os.path.exists(REF_BIN) or not os.path.exists(os.path.join(simt_emu.ROOT, "oracle", "_ref", "obj", "main.o"))
+                    or not simt_emu.REF_SRC or not os.path.exists(os.path.join(simt_emu.REF_SRC, "main.cpp")),
+                    reason="oracle/_ref (the reference's objects and binary) not built, or the reference's headers absent")
 @pytest.mark.parametrize("flags,threads", [(["--cut_front", "--cut_tail", "-x", "-y"], 3), (["-N", "-b", "-s", synth.ADAPTER_START], 2)])
 def test_emulated_drop_in_binary_writes_the_reference_binary_s_files(flags, threads, tmp_path):
     exe = simt_emu.build_binary()

@@ -1,7 +1,6 @@
 """Adapter auto-detection (SURVEY §8f row 4): fastplong_b200/evaluator.py (host half) against the unmodified reference
 binary's own detection, and the device ten-mer tables against their numpy restatement."""
 import json
-import os
 import subprocess
 
 import numpy as np
@@ -9,6 +8,7 @@ import pytest
 
 from fastplong_b200 import evaluator, synth
 from oracle_lib import REF_BIN, kmer10_tables
+from reference_outputs import digest, expected
 
 
 def reference_detection(batch, tmp_path, extra=()):
@@ -23,17 +23,23 @@ def reference_detection(batch, tmp_path, extra=()):
     return ac.get("read_start_adapter"), ac.get("read_end_adapter"), r.stderr
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 @pytest.mark.parametrize("seed,kw", [(5, {}), (6, dict(p_start=0.5, p_end=0.9)), (7, dict(p_start=0.05, p_end=0.6)),
                                      (8, dict(adapter_start="GATCGGAAGAGCACACGTCTGAACTCCAGTCAC", adapter_end="ACACTCTTTCCCTACACGACGCTCTTCCGATCT"))])
 def test_host_logic_matches_reference_binary(seed, kw, tmp_path):
+    """The adapters the reference binary detected on these seeded reads (stored, tests/reference_outputs.py)."""
     batch = synth.ont_like(600, 1500, seed, **kw)
-    start, end, log = reference_detection(batch, tmp_path)
+    inp = digest(np.concatenate([batch.seq, batch.qual]))
+    def run_reference():
+        start, end, _ = reference_detection(batch, tmp_path)
+        return {"input": inp, "start": start, "end": end}
+    ref = expected(f"evaluator/{seed}", run_reference)
+    assert ref["input"] == inp, "the seeded reads are not the ones the reference ran on"
+    start, end = ref["start"], ref["end"]
     # the JSON prints "unspecified" for an adapter left at "auto" (src/options.cpp:247-259)
     norm = lambda s: "unspecified" if s == "auto" else s
     for pick in ("abi", "python"):       # the C ABI's fpl_eval_pick_adapter and its Python twin
         got = evaluator.detect_adapters(batch, kmers=kmer10_tables, pick=pick)
-        assert (norm(got[0]), norm(got[1])) == (start, end), (pick, log[-600:])
+        assert (norm(got[0]), norm(got[1])) == (start, end), pick
 
 
 def _planted_tables(rng):

@@ -1,6 +1,7 @@
 """Whole-binary parity: build/fastplong_gpu (the reference CLI with our SingleEndProcessor + libfplgpu.so) against
-oracle/_ref/fastplong_ref (the unmodified reference) and against the committed golden runs: md5 of --out and
---failed_out, and the JSON report text minus its "command" line (SURVEY §8c)."""
+what oracle/_ref/fastplong_ref (the unmodified reference) wrote for the same seeded inputs (stored,
+tests/reference_outputs.py) and against the committed golden runs: md5 of --out and --failed_out, and the JSON report
+text minus its "command" line (SURVEY §8c)."""
 import hashlib
 import json
 import os
@@ -11,6 +12,7 @@ import pytest
 import cases
 from fastplong_b200 import synth
 from oracle_lib import REF_BIN
+from reference_outputs import expected
 
 pytestmark = pytest.mark.gpu
 
@@ -40,6 +42,14 @@ def run(binary, opt, fq, outdir, tag, threads=3, extra=(), env=None):
     return {"out_md5": md5(out), "failed_md5": md5(failed), "json_text_md5": json_text_md5(js), "json": js}
 
 
+def reference_run(key, opt, fq, outdir, threads, extra=()):
+    """The md5s of what the reference binary wrote for this input and these options."""
+    inp = md5(fq)
+    ref = expected("binary/" + key, lambda: dict(run(REF_BIN, opt, fq, outdir, "ref", threads, extra), json=None, input_md5=inp))
+    assert ref["input_md5"] == inp, f"{key}: the seeded input is not the one the reference ran on"
+    return ref
+
+
 needs_bin = pytest.mark.skipif(not os.path.exists(GPU_BIN), reason="build/fastplong_gpu not built")
 
 
@@ -59,7 +69,6 @@ def test_gpu_binary_matches_golden_reference_run(name, tmp_path):
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 @pytest.mark.parametrize("parse", ["device", "host", "device+emit"])
 @pytest.mark.parametrize("name,threads", [("default_se", 1), ("cut_polyx_cplx", 4), ("fasta5", 3), ("literal_auto", 2),
                                           ("trims_limits", 3), ("end_only_wide_window", 8), ("fasta64_polyx", 5)])
@@ -78,16 +87,11 @@ def test_gpu_binary_matches_reference_binary(name, threads, parse, tmp_path):
             for i, s in enumerate(opt.adapter_fasta):
                 f.write(f">a{i:03d}\n{s}\n")
         extra = ["-a", fa]
-    ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", threads, extra)
+    ref = reference_run(f"{name}/w{threads}", opt, fq, str(tmp_path), threads, extra)
     got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", threads, extra, env=PARSE_ENV[parse])
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
-    if got["json_text_md5"] != ref["json_text_md5"]:
-        a, b = json.load(open(got["json"])), json.load(open(ref["json"]))
-        a.pop("command"); b.pop("command")
-        for k in b:
-            assert a[k] == b[k], k
-        raise AssertionError("JSON text differs although the parsed content is equal")
+    assert got["json_text_md5"] == ref["json_text_md5"]
 
 
 @needs_bin
@@ -106,7 +110,6 @@ def test_gpu_binary_mask_break_matches_golden_reference_run(name, tmp_path):
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 @pytest.mark.parametrize("parse", ["device", "host", "device+emit"])
 @pytest.mark.parametrize("name,threads", [("break_default", 2), ("break_w20", 3), ("mask_default", 1), ("mask_cplx", 4),
                                           ("mask_and_break", 3), ("break_no_adapter", 2)])
@@ -116,7 +119,7 @@ def test_gpu_binary_mask_break_matches_reference_binary(name, threads, parse, tm
     batch = cases.blocky_quality_batch(40 + threads, n=400)
     fq = str(tmp_path / "in.fq")
     synth.to_fastq(batch, fq)
-    ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", threads)
+    ref = reference_run(f"mb/{name}/w{threads}", opt, fq, str(tmp_path), threads)
     got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", threads, env=PARSE_ENV[parse])
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
@@ -124,18 +127,16 @@ def test_gpu_binary_mask_break_matches_reference_binary(name, threads, parse, tm
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 def test_config1_full_size_bit_exact(tmp_path):
     """BASELINE configs[0] at full size: 10k ONT reads mean 8 kb, known 30 bp start/end adapters, default Q-filter —
-    reference CPU run vs the GPU binary, bit-exact FASTQ outputs and JSON report; prints both wall times."""
+    the reference CPU run's outputs vs the GPU binary, bit-exact FASTQ outputs and JSON report; prints the GPU wall times."""
     import time
     opt = cases.OPTION_SETS["default_se"]
     batch = synth.ont_like(10000, 8000, 1)
-    fq = "/dev/shm/fpl_c1.fq" if os.path.isdir("/dev/shm") else str(tmp_path / "c1.fq")
+    fq = "/dev/shm/fpl_c1_%d.fq" % os.getpid() if os.path.isdir("/dev/shm") else str(tmp_path / "c1.fq")
     synth.to_fastq(batch, fq)
     try:
-        t0 = time.perf_counter()
-        ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", threads=16)
+        ref = reference_run("config1", opt, fq, str(tmp_path), 16)
         t1 = time.perf_counter()
         got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", threads=4)
         t2 = time.perf_counter()
@@ -144,13 +145,9 @@ def test_config1_full_size_bit_exact(tmp_path):
     finally:
         if fq.startswith("/dev/shm"):
             os.remove(fq)
-    print(f"\nconfig 1 ({batch.n_bases / 1e6:.1f} Mbases): fastplong_ref -w 16 {t1 - t0:.2f} s, fastplong_gpu -w 4 {t2 - t1:.2f} s "
-          f"(device FASTQ parse), {t3 - t2:.2f} s (reference reader)")
+    print(f"\nconfig 1 ({batch.n_bases / 1e6:.1f} Mbases): fastplong_gpu -w 4 {t2 - t1:.2f} s (device FASTQ parse), "
+          f"{t3 - t2:.2f} s (reference reader)")
     assert got_host["out_md5"] == ref["out_md5"] and got_host["json_text_md5"] == ref["json_text_md5"]
-    open(os.path.join(ROOT, "gpurun_out", "c1_binary_times.txt"), "w").write(
-        f"config1 {batch.n_reads} reads {batch.n_bases} bases ref_w16_s {t1 - t0:.3f} gpu_w4_device_parse_s {t2 - t1:.3f} "
-        f"gpu_w4_host_parse_s {t3 - t2:.3f}\n") \
-        if os.path.isdir(os.path.join(ROOT, "gpurun_out")) else None
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
     assert got["json_text_md5"] == ref["json_text_md5"]
@@ -178,7 +175,6 @@ def _mutate_fastq(src, dst, kind):
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 @pytest.mark.parametrize("kind", ["crlf", "blank_line_mid", "cr_mid", "blank_line_eof", "truncated_last_record",
                                   "stray_line_between_records"])
 def test_gpu_binary_non_strict_fastq_like_reference(kind, tmp_path):
@@ -190,7 +186,7 @@ def test_gpu_binary_non_strict_fastq_like_reference(kind, tmp_path):
     plain, fq = str(tmp_path / "plain.fq"), str(tmp_path / "in.fq")
     synth.to_fastq(batch, plain)
     _mutate_fastq(plain, fq, kind)
-    ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", 3)
+    ref = reference_run(f"non_strict/{kind}", opt, fq, str(tmp_path), 3)
     got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", 3)
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
@@ -198,7 +194,6 @@ def test_gpu_binary_non_strict_fastq_like_reference(kind, tmp_path):
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 @pytest.mark.parametrize("emit", ["host", "device"])
 @pytest.mark.parametrize("chunk_kb,threads", [(256, 4), (64, 7), (1, 2)])
 def test_gpu_binary_many_small_chunks(chunk_kb, threads, emit, tmp_path):
@@ -212,7 +207,7 @@ def test_gpu_binary_many_small_chunks(chunk_kb, threads, emit, tmp_path):
     env = {"FPL_CHUNK_KB": str(chunk_kb), "FPL_WRITER_BACKLOG": "1"}
     if emit == "device":
         env["FPL_DEVICE_EMIT"] = "1"
-    ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", threads)
+    ref = reference_run(f"chunks/{chunk_kb}kb/w{threads}", opt, fq, str(tmp_path), threads)
     got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", threads, env=env)
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
@@ -220,7 +215,6 @@ def test_gpu_binary_many_small_chunks(chunk_kb, threads, emit, tmp_path):
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 def test_gpu_binary_file_size_is_a_multiple_of_the_chunk(tmp_path):
     """The last fread returns 0 bytes: the final chunk is whatever was left over (possibly nothing)."""
     opt = cases.OPTION_SETS["default_se"]
@@ -233,7 +227,7 @@ def test_gpu_binary_file_size_is_a_multiple_of_the_chunk(tmp_path):
     with open(fq, "ab") as f:
         f.write(b"@p" + b"x" * pad + b"\nACGTACGTAC\n+\nIIIIIIIIII\n")
     assert os.path.getsize(fq) % unit == 0
-    ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", 3)
+    ref = reference_run("chunk_multiple", opt, fq, str(tmp_path), 3)
     got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", 3, env={"FPL_CHUNK_KB": "64"})
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
@@ -241,7 +235,6 @@ def test_gpu_binary_file_size_is_a_multiple_of_the_chunk(tmp_path):
 
 
 @needs_bin
-@pytest.mark.skipif(not os.path.exists(REF_BIN), reason="oracle/_ref/fastplong_ref not built")
 @pytest.mark.parametrize("emit", ["host", "device"])
 def test_gpu_binary_plus_lines_kept_verbatim(emit, tmp_path):
     """The third line of a record may repeat the name ('+name ...'): Read::appendToString writes it back as it was
@@ -255,7 +248,7 @@ def test_gpu_binary_plus_lines_kept_verbatim(emit, tmp_path):
             name = b"@read%d len=%d" % (i, len(s))
             plus = b"+" if i % 3 == 0 else (b"+" + name[1:] if i % 3 == 1 else b"+ free text %d" % i)
             f.write(name + b"\n" + s + b"\n" + plus + b"\n" + q + b"\n")
-    ref = run(REF_BIN, opt, fq, str(tmp_path), "ref", 3)
+    ref = reference_run("plus_lines", opt, fq, str(tmp_path), 3)
     got = run(GPU_BIN, opt, fq, str(tmp_path), "gpu", 3, env={"FPL_DEVICE_EMIT": "1"} if emit == "device" else None)
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]

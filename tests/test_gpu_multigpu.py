@@ -36,21 +36,20 @@ def test_two_gpu_shard_merge_gather(optset):
                                               ("default_se", 5, {"FPL_HOST_PARSE": "1"})])
 def test_drop_in_binary_workers_over_two_gpus(name, threads, env, tmp_path):
     """build/fastplong_gpu spreads its worker contexts over the visible devices (worker t -> device t mod 2) and the
-    reference's own Stats::merge adds them on the host: outputs and JSON must equal the reference binary's."""
+    reference's own Stats::merge adds them on the host: outputs and JSON must equal the reference binary's (stored)."""
     if _n_gpus() < 2:
         pytest.skip("needs 2 GPUs")
     sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
     import cases
     import test_gpu_binary as tb
     from fastplong_b200 import synth
-    from oracle_lib import REF_BIN
-    if not (os.path.exists(tb.GPU_BIN) and os.path.exists(REF_BIN)):
-        pytest.skip("binaries not built")
+    if not os.path.exists(tb.GPU_BIN):
+        pytest.skip("build/fastplong_gpu not built")
     opt = cases.OPTION_SETS.get(name) or cases.MASK_BREAK_SETS[name]
     batch = synth.ont_like(3000, 5000, 77, p_chimera=0.03, p_polya=0.03, q_mean=17.0)    # several chunks per worker
     fq = str(tmp_path / "in.fq")
     synth.to_fastq(batch, fq)
-    ref = tb.run(REF_BIN, opt, fq, str(tmp_path), "ref", threads)
+    ref = tb.reference_run(f"two_gpus/{name}/w{threads}", opt, fq, str(tmp_path), threads)
     got = tb.run(tb.GPU_BIN, opt, fq, str(tmp_path), "gpu", threads, env=dict(env or {}, FPL_TIMING="1"))
     assert got["out_md5"] == ref["out_md5"]
     assert got["failed_md5"] == ref["failed_md5"]
