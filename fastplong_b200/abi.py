@@ -2,7 +2,7 @@
 import ctypes as C
 import numpy as np
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 COMM_ID_BYTES = 128        # FPL_COMM_ID_BYTES == sizeof(ncclUniqueId)
 MAX_ADAPTER_LEN = 1024
 MAX_ADAPTERS = 1024
@@ -30,6 +30,13 @@ def stats_words(cycles):
 
 def counter_words(n_adapters):
     return CNT_FIXED + int(n_adapters) * 2 * (MAX_ADAPTER_LEN + 1)
+
+GZIP_SEGMENT = 65536       # FPL_GZIP_SEGMENT
+
+
+def gzip_bound(n_bytes, n_pieces):
+    """FPL_GZIP_BOUND: the most bytes fpl_gzip_host writes for n_bytes in n_pieces pieces."""
+    return int(n_bytes) + 28 * (int(n_bytes) // GZIP_SEGMENT + int(n_pieces))
 
 
 def event_unpack(e):

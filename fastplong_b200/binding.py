@@ -38,6 +38,8 @@ def load_library():
                                            C.POINTER(C.c_int64), C.POINTER(C.c_int64)]
     lib.fpl_emit_fastq_host.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.c_void_p, C.c_int64,
                                         C.POINTER(C.c_int64)]
+    lib.fpl_gzip_host.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.fpl_emit_fastq_gzip_host.argtypes = lib.fpl_emit_fastq_host.argtypes
     lib.fpl_stream.argtypes = [C.c_void_p]
     lib.fpl_stream.restype = C.c_void_p
     lib.fpl_fetch_results.argtypes = [C.c_void_p, C.c_void_p, C.c_int64]
@@ -74,7 +76,7 @@ def load_library():
 
 
 EXPORTS = ["fpl_last_error", "fpl_abi_version", "fpl_create", "fpl_destroy", "fpl_process_host", "fpl_process_device", "fpl_process_fastq_host", "fpl_emit_fastq_host",
-           "fpl_sync", "fpl_stream", "fpl_last_segments", "fpl_last_mask_regions", "fpl_fetch_results", "fpl_stats_cycles", "fpl_stats_reserve", "fpl_stats_download",
+           "fpl_gzip_host", "fpl_emit_fastq_gzip_host", "fpl_sync", "fpl_stream", "fpl_last_segments", "fpl_last_mask_regions", "fpl_fetch_results", "fpl_stats_cycles", "fpl_stats_reserve", "fpl_stats_download",
            "fpl_stats_device_ptr", "fpl_counter_words", "fpl_counters_download", "fpl_counters_device_ptr",
            "fpl_comm_unique_id", "fpl_comm_init", "fpl_comm_destroy", "fpl_comm_size", "fpl_comm_agree_cycles", "fpl_allreduce_stats",
            "fpl_eval_adapter_kmers", "fpl_eval_pick_adapter", "fpl_reset", "fpl_last_kernel_times", "fpl_launch_count", "fpl_set_timing"]
@@ -147,16 +149,36 @@ class Engine:
     def emit_fastq(self, want_failed=True):
         """The --out / --failed_out text of the chunk the last process_fastq() call processed, assembled on the device
         (fpl_emit_fastq_host): (out_bytes, failed_bytes).  First call sizes, second call copies."""
+        return self._emit(self.lib.fpl_emit_fastq_host, want_failed)
+
+    def _emit(self, fn, want_failed):
         n_out, n_failed = C.c_int64(), C.c_int64()
-        rc = self.lib.fpl_emit_fastq_host(self.h, int(want_failed), None, 0, C.byref(n_out), None, 0, C.byref(n_failed))
+        rc = fn(self.h, int(want_failed), None, 0, C.byref(n_out), None, 0, C.byref(n_failed))
         if rc < 0:
             self._check(rc)
         out = np.empty(n_out.value, dtype=np.uint8)
         failed = np.empty(n_failed.value, dtype=np.uint8)
-        self._check(self.lib.fpl_emit_fastq_host(self.h, int(want_failed), out.ctypes.data if out.size else None, out.size,
-                                                 C.byref(n_out), failed.ctypes.data if failed.size else None, failed.size,
-                                                 C.byref(n_failed)))
+        self._check(fn(self.h, int(want_failed), out.ctypes.data if out.size else None, out.size, C.byref(n_out),
+                       failed.ctypes.data if failed.size else None, failed.size, C.byref(n_failed)))
         return out.tobytes(), failed.tobytes()
+
+    def emit_fastq_gzip(self, want_failed=True):
+        """emit_fastq() with both texts compressed on the device (fpl_emit_fastq_gzip_host): (out_gz, failed_gz), each a
+        multi-member gzip stream."""
+        return self._emit(self.lib.fpl_emit_fastq_gzip_host, want_failed)
+
+    def gzip(self, pieces):
+        """Each piece (bytes-like) compressed on the device into gzip members (fpl_gzip_host) -> list of bytes."""
+        bufs = [bytes(p) for p in pieces]
+        text = np.frombuffer(b"".join(bufs), dtype=np.uint8)
+        sizes = np.array([len(b) for b in bufs], dtype=np.int64)
+        cap = abi.gzip_bound(text.size, len(bufs))
+        out = np.empty(max(cap, 1), dtype=np.uint8)
+        out_sizes = np.zeros(max(len(bufs), 1), dtype=np.int64)
+        self._check(self.lib.fpl_gzip_host(self.h, text.ctypes.data if text.size else None, sizes.ctypes.data, len(bufs),
+                                           out.ctypes.data, cap, out_sizes.ctypes.data))
+        ends = np.cumsum(out_sizes[:len(bufs)])
+        return [out[e - k:e].tobytes() for e, k in zip(ends, out_sizes[:len(bufs)])]
 
     def process_device(self, seq_ptr, qual_ptr, offsets_ptr, lens_ptr, n_reads, n_bytes, results_ptr=None):
         b = FplBatch(seq_ptr, qual_ptr, offsets_ptr, lens_ptr, n_reads, n_bytes)

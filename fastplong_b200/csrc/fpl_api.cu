@@ -20,6 +20,7 @@
 #include "fpl_ingest.h"
 #include "fpl_ext.h"
 #include "fpl_emit.h"
+#include "fpl_gzip.h"
 
 static_assert(sizeof(fpl_options) == 144, "fpl_options ABI size");
 static_assert(sizeof(fpl_segment) == 20 && sizeof(fpl_region) == 12, "segment / region ABI size");
@@ -55,11 +56,11 @@ static int fail(const char* fmt, ...) {
         if (e_ != cudaSuccess) return fail("%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
     } while (0)
 
-enum { K_PRESEG, K_CYCLE_PRE, K_QUAL_PRE, K_TRIM, K_SCAN, K_FINAL, K_COUNT, K_CYCLE_POST, K_QUAL_POST, K_KMER_FIX, K_ALLREDUCE, K_NKERNELS };
+enum { K_PRESEG, K_CYCLE_PRE, K_QUAL_PRE, K_TRIM, K_SCAN, K_FINAL, K_COUNT, K_CYCLE_POST, K_QUAL_POST, K_KMER_FIX, K_ALLREDUCE, K_GZ_DEFLATE, K_GZ_COMPACT, K_NKERNELS };
 static const char* const kKernelNames[K_NKERNELS] = {"k_make_preseg", "k_cycle_stats(pre)", "k_read_qual(pre+post)",
                                                      "k_trim", "k_scan", "k_final", "k_count",
                                                      "k_cycle_stats(post)", "k_read_qual(post)", "k_kmer_fix",
-                                                     "nccl_allreduce(stats)"};
+                                                     "nccl_allreduce(stats)", "k_gzip_deflate", "k_gzip_compact"};
 
 struct fpl_ctx {
     int device = 0;
@@ -71,6 +72,10 @@ struct fpl_ctx {
     FplExt ext;         // --mask / --break state (variable number of output reads)
     FplEmit emit;       // device-side output text of the last fpl_process_fastq_host chunk (fpl_emit_fastq_host)
     bool emit_valid = false;            // the last call was a successful fpl_process_fastq_host: chunk + records + results in HBM
+    FplGzip gz;         // device gzip encoder state (fpl_gzip_host, fpl_emit_fastq_gzip_host)
+    bool emit_gz_built = false;         // gz.d_out holds the compressed emit text (out piece, then failed piece)
+    bool emit_gz_failed = false;
+    int64_t emit_gz_bytes[2] = {0, 0};
     int64_t emit_n = 0;
     int64_t last_bytes = 0;
     bool slots16 = false;               // this batch's read offsets are multiples of 16 (checked: host batches, device ingest)
@@ -221,7 +226,7 @@ static int run_batch(fpl_ctx* c, const DevBatch& full, const int32_t* h_lens, fp
     const int64_t n = full.n_reads;
     CK(cudaSetDevice(c->device));
     collect_times(c);
-    c->emit_valid = false; c->emit.built = false;
+    c->emit_valid = false; c->emit.built = false; c->emit_gz_built = false;
     c->last_n = n;
     if (ensure_reads(c, n)) return -1;
     fpl_read_result* d_res = d_res_out ? d_res_out : c->d_results;
@@ -513,6 +518,7 @@ void fpl_destroy(fpl_ctx* c) {
     fpl_ingest_free(&c->ingest);
     fpl_ext_free(&c->ext);
     fpl_emit_free(&c->emit);
+    fpl_gzip_free(&c->gz);
     if (c->stream) cudaStreamDestroy(c->stream);
     delete c;
 }
@@ -648,7 +654,7 @@ int fpl_process_fastq_host(fpl_ctx* c, const uint8_t* text, int64_t n_bytes, int
     if (rc < 0) return fail("fpl_process_fastq_host: %s", err);
     if (rc > 0) return 1;
     *n_records = nrec;
-    c->emit_valid = false; c->emit.built = false;
+    c->emit_valid = false; c->emit.built = false; c->emit_gz_built = false;
     if (nrec == 0) { c->emit_valid = true; c->emit_n = 0; return 0; }
     if (nrec > max_records) return 1;
     if (!records || !results) return fail("fpl_process_fastq_host: records/results is null");
@@ -678,13 +684,10 @@ int fpl_process_fastq_host(fpl_ctx* c, const uint8_t* text, int64_t n_bytes, int
     return 0;
 }
 
-int fpl_emit_fastq_host(fpl_ctx* c, int want_failed, uint8_t* out, int64_t out_cap, int64_t* out_bytes, uint8_t* failed,
-                        int64_t failed_cap, int64_t* failed_bytes) {
-    g_err[0] = 0;
-    if (!c || !out_bytes || !failed_bytes) return fail("fpl_emit_fastq_host: null argument");
-    *out_bytes = *failed_bytes = 0;
+// Builds the emit text of the last chunk on the device unless it is built already (for the same want_failed).
+static int ensure_emit(fpl_ctx* c, int want_failed, const char* fn) {
     if (!c->emit_valid)
-        return fail("fpl_emit_fastq_host: the last call on this context was not a successful fpl_process_fastq_host");
+        return fail("%s: the last call on this context was not a successful fpl_process_fastq_host", fn);
     CK(cudaSetDevice(c->device));
     FplEmit& e = c->emit;
     if (!e.built || e.with_failed != (want_failed != 0)) {
@@ -696,15 +699,96 @@ int fpl_emit_fastq_host(fpl_ctx* c, int want_failed, uint8_t* out, int64_t out_c
         src.mseq = (c->P.opt.mask_enabled && c->ext.n_segs > 0) ? c->ext.d_mseq : nullptr;   // fpl_ext_run made the masked copy
         src.offsets = c->ingest.d_offsets;
         char err[256] = "";
-        if (fpl_emit_build(&e, src, want_failed != 0, c->stream, err, sizeof(err))) return fail("fpl_emit_fastq_host: %s", err);
+        c->emit_gz_built = false;
+        if (fpl_emit_build(&e, src, want_failed != 0, c->stream, err, sizeof(err))) return fail("%s: %s", fn, err);
         if (c->emit_n) c->launches += 2;
     }
+    return 0;
+}
+
+int fpl_emit_fastq_host(fpl_ctx* c, int want_failed, uint8_t* out, int64_t out_cap, int64_t* out_bytes, uint8_t* failed,
+                        int64_t failed_cap, int64_t* failed_bytes) {
+    g_err[0] = 0;
+    if (!c || !out_bytes || !failed_bytes) return fail("fpl_emit_fastq_host: null argument");
+    *out_bytes = *failed_bytes = 0;
+    if (ensure_emit(c, want_failed, "fpl_emit_fastq_host")) return -1;
+    FplEmit& e = c->emit;
     *out_bytes = e.out_bytes;
     *failed_bytes = e.failed_bytes;
     if (e.out_bytes > out_cap || e.failed_bytes > failed_cap) return 1;     // the text stays built: call again with room
     if ((e.out_bytes && !out) || (e.failed_bytes && !failed)) return fail("fpl_emit_fastq_host: null output buffer");
     if (e.out_bytes) CK(cudaMemcpyAsync(out, e.d_out, (size_t)e.out_bytes, cudaMemcpyDeviceToHost, c->stream));
     if (e.failed_bytes) CK(cudaMemcpyAsync(failed, e.d_failed, (size_t)e.failed_bytes, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+// Compresses device-resident pieces into c->gz.d_out (back to back); piece_out[i] = compressed bytes of piece i.
+static int gzip_pieces(fpl_ctx* c, const uint8_t* const* piece, const int64_t* bytes, int n_pieces, int64_t* piece_out,
+                       const char* fn) {
+    char err[256] = "";
+    collect_times(c);
+    if (fpl_gzip_plan(&c->gz, piece, bytes, n_pieces, c->stream, err, sizeof(err))) return fail("%s: %s", fn, err);
+    if (c->gz.n_segs) {
+        { Timed t(c, K_GZ_DEFLATE); fpl_gzip_deflate(&c->gz, c->stream); }
+        CK(cudaGetLastError());
+        if (fpl_gzip_offsets(&c->gz, c->stream, err, sizeof(err))) return fail("%s: %s", fn, err);
+        { Timed t(c, K_GZ_COMPACT); fpl_gzip_compact(&c->gz, c->stream); }
+        CK(cudaGetLastError());
+    }
+    if (fpl_gzip_piece_sizes(&c->gz, piece_out, c->stream, err, sizeof(err))) return fail("%s: %s", fn, err);
+    collect_times(c);
+    return 0;
+}
+
+int fpl_gzip_host(fpl_ctx* c, const uint8_t* text, const int64_t* piece_bytes, int32_t n_pieces, uint8_t* out, int64_t out_cap,
+                  int64_t* out_piece_bytes) {
+    g_err[0] = 0;
+    if (!c || n_pieces < 0 || (n_pieces > 0 && (!piece_bytes || !out_piece_bytes))) return fail("fpl_gzip_host: bad argument");
+    int64_t total = 0;
+    for (int i = 0; i < n_pieces; i++) {
+        if (piece_bytes[i] < 0) return fail("fpl_gzip_host: piece %d has a negative size", i);
+        total += piece_bytes[i];
+    }
+    if ((total && !text) || out_cap < FPL_GZIP_BOUND(total, n_pieces) || (FPL_GZIP_BOUND(total, n_pieces) > 0 && !out))
+        return fail("fpl_gzip_host: the output buffer holds %lld bytes, FPL_GZIP_BOUND(%lld, %d) = %lld", (long long)out_cap,
+                    (long long)total, n_pieces, (long long)FPL_GZIP_BOUND(total, n_pieces));
+    CK(cudaSetDevice(c->device));
+    c->emit_gz_built = false;                           // gz.d_out is about to be overwritten
+    char err[256] = "";
+    if (fpl_gzip_grow((void**)&c->gz.d_in, &c->gz.cap_in, total + 16, err, sizeof(err))) return fail("fpl_gzip_host: %s", err);
+    if (total) CK(cudaMemcpyAsync(c->gz.d_in, text, (size_t)total, cudaMemcpyHostToDevice, c->stream));
+    std::vector<const uint8_t*> ptr((size_t)n_pieces);
+    for (int64_t i = 0, o = 0; i < n_pieces; o += piece_bytes[i], i++) ptr[(size_t)i] = c->gz.d_in + o;
+    if (gzip_pieces(c, ptr.data(), piece_bytes, n_pieces, out_piece_bytes, "fpl_gzip_host")) return -1;
+    int64_t n_out = 0;
+    for (int i = 0; i < n_pieces; i++) n_out += out_piece_bytes[i];
+    if (n_out) CK(cudaMemcpyAsync(out, c->gz.d_out, (size_t)n_out, cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int fpl_emit_fastq_gzip_host(fpl_ctx* c, int want_failed, uint8_t* out, int64_t out_cap, int64_t* out_bytes, uint8_t* failed,
+                             int64_t failed_cap, int64_t* failed_bytes) {
+    g_err[0] = 0;
+    if (!c || !out_bytes || !failed_bytes) return fail("fpl_emit_fastq_gzip_host: null argument");
+    *out_bytes = *failed_bytes = 0;
+    if (ensure_emit(c, want_failed, "fpl_emit_fastq_gzip_host")) return -1;
+    FplEmit& e = c->emit;
+    if (!c->emit_gz_built || c->emit_gz_failed != (want_failed != 0)) {
+        const uint8_t* piece[2] = {e.d_out, e.d_failed};
+        const int64_t bytes[2] = {e.out_bytes, e.failed_bytes};
+        if (gzip_pieces(c, piece, bytes, 2, c->emit_gz_bytes, "fpl_emit_fastq_gzip_host")) return -1;
+        c->emit_gz_built = true;
+        c->emit_gz_failed = want_failed != 0;
+    }
+    *out_bytes = c->emit_gz_bytes[0];
+    *failed_bytes = c->emit_gz_bytes[1];
+    if (*out_bytes > out_cap || *failed_bytes > failed_cap) return 1;      // stays compressed on the device: call again with room
+    if ((*out_bytes && !out) || (*failed_bytes && !failed)) return fail("fpl_emit_fastq_gzip_host: null output buffer");
+    if (*out_bytes) CK(cudaMemcpyAsync(out, c->gz.d_out, (size_t)*out_bytes, cudaMemcpyDeviceToHost, c->stream));
+    if (*failed_bytes)
+        CK(cudaMemcpyAsync(failed, c->gz.d_out + *out_bytes, (size_t)*failed_bytes, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     return 0;
 }

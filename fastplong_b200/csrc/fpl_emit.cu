@@ -217,3 +217,7 @@ void fpl_emit_free(FplEmit* e) {
     cudaFree(e->d_size); cudaFree(e->d_off); cudaFree(e->d_out); cudaFree(e->d_failed); cudaFree(e->d_tmp);
     *e = FplEmit();
 }
+
+// The gzip encoder that compresses this text (fpl_emit_fastq_gzip_host) and any other (fpl_gzip_host) is compiled in
+// this translation unit.
+#include "fpl_gzip.cuh"

@@ -33,10 +33,13 @@
 
 // Stats / FilterResult keep their accumulators private and offer no setters (src/stats.h:56-113,
 // src/filterresult.h:58-64); this adapter TU is compiled with the class keys opened so that it can ADD the
-// device-accumulated arrays into them.  The reference's own TUs are compiled untouched.
+// device-accumulated arrays into them.  The reference's own TUs are compiled untouched.  Writer / WriterThread are opened
+// the same way so that FPL_DEVICE_GZIP can switch a writer's own compression off (see switchWriterToDeviceGzip).
 #define private public
 #include "stats.h"
 #include "filterresult.h"
+#include "writer.h"
+#include "writerthread.h"
 #undef private
 #include "seprocessor.h"
 #include "fastqreader.h"
@@ -387,10 +390,53 @@ SingleEndProcessor::~SingleEndProcessor() {
     delete[] mInputLists;
 }
 
+// FPL_DEVICE_GZIP=1: a writer whose file name ends in ".gz" no longer compresses (Writer::writeInternal's
+// libdeflate_gzip_compress, src/writer.cpp:110-126, on the single writer thread); the workers hand it strings that are
+// already whole gzip members, compressed on the device, and it only writes them.  Members may be concatenated at any
+// buffer boundary, so the file stays one valid multi-member gzip stream.  --split and --stdout ignore the knob.
+static bool g_gzLeft = false, g_gzFailed = false;   // the workers compress the --out / --failed_out strings
+
+static bool switchWriterToDeviceGzip(WriterThread* wt, Options* opt) {
+    if (!wt || !getenv("FPL_DEVICE_GZIP") || opt->split.enabled || wt->mWriter1 == NULL || wt->mWriter1->mSTDOUT ||
+        !ends_with(wt->mFilename, ".gz"))
+        return false;
+    Writer* w = wt->mWriter1;
+    if (w->mZipped) {
+        libdeflate_free_compressor(w->mCompressor);
+        w->mCompressor = NULL;
+        w->mZipped = false;
+    }
+    return true;
+}
+
+// Compresses the non-null strings in place on the device, each into whole gzip members: one fpl_gzip_host call for all.
+static void gzipStrings(fpl_ctx* ctx, const std::vector<std::string*>& strs) {
+    thread_local Pinned<uint8_t> in, out;
+    thread_local std::vector<int64_t> sizes, outSizes;
+    sizes.clear();
+    size_t total = 0;
+    for (std::string* s : strs) if (s) { sizes.push_back((int64_t)s->size()); total += s->size(); }
+    if (sizes.empty()) return;
+    const int64_t bound = FPL_GZIP_BOUND((int64_t)total, (int64_t)sizes.size());
+    in.reserve(total + 1, 1u << 20);
+    out.reserve((size_t)bound + 1, 1u << 20);
+    size_t o = 0;
+    for (std::string* s : strs) if (s) { memcpy(in.p + o, s->data(), s->size()); o += s->size(); }
+    outSizes.assign(sizes.size(), 0);
+    check(fpl_gzip_host(ctx, in.p, sizes.data(), (int32_t)sizes.size(), out.p, bound, outSizes.data()), "fpl_gzip_host");
+    size_t k = 0;
+    o = 0;
+    for (std::string* s : strs)
+        if (s) { s->assign((const char*)out.p + o, (size_t)outSizes[k]); o += (size_t)outSizes[k]; k++; }
+}
+
 void SingleEndProcessor::initOutput() {
     if (!mOptions->failedOut.empty()) mFailedWriter = new WriterThread(mOptions, mOptions->failedOut);
+    g_gzFailed = switchWriterToDeviceGzip(mFailedWriter, mOptions);
+    g_gzLeft = false;
     if (mOptions->out.empty() && !mOptions->outputToSTDOUT) return;
     mLeftWriter = new WriterThread(mOptions, mOptions->out, mOptions->outputToSTDOUT);
+    g_gzLeft = switchWriterToDeviceGzip(mLeftWriter, mOptions);
 }
 
 void SingleEndProcessor::closeOutput() {
@@ -500,6 +546,9 @@ bool SingleEndProcessor::processSingleEnd(ReadPack* pack, ThreadConfig* config) 
     ext.fetch(w.ctx, mOptions->mask.enabled || mOptions->breakOpt.enabled);
     std::string scratch;
     k = 0;
+    // FPL_DEVICE_GZIP: the batch's strings are compressed together (one device call) and then handed on in pack order
+    const bool gz = (mLeftWriter && g_gzLeft) || (mFailedWriter && g_gzFailed);
+    std::vector<std::pair<string*, string*>> held;
     for (ReadPack* p : w.packs) {
         string* outstr = new string();
         string* failedOut = new string();
@@ -518,8 +567,13 @@ bool SingleEndProcessor::processSingleEnd(ReadPack* pack, ThreadConfig* config) 
         if (mOptions->split.enabled) {
             if (!mOptions->out.empty()) config->getWriter1()->writeString(outstr);
         }
-        if (mLeftWriter) { mLeftWriter->input(tid, outstr); outstr = NULL; }
-        if (mFailedWriter) { mFailedWriter->input(tid, failedOut); failedOut = NULL; }
+        if (gz) {
+            held.emplace_back(mLeftWriter ? outstr : NULL, mFailedWriter ? failedOut : NULL);
+            if (mLeftWriter) outstr = NULL;
+            if (mFailedWriter) failedOut = NULL;
+        }
+        if (mLeftWriter && outstr) { mLeftWriter->input(tid, outstr); outstr = NULL; }
+        if (mFailedWriter && failedOut) { mFailedWriter->input(tid, failedOut); failedOut = NULL; }
         if (mOptions->split.byFileLines) config->markProcessed(readPassed);
         else config->markProcessed(p->count);
         delete outstr;
@@ -528,6 +582,18 @@ bool SingleEndProcessor::processSingleEnd(ReadPack* pack, ThreadConfig* config) 
         delete p;
     }
     w.packs.clear();
+    if (gz) {
+        std::vector<std::string*> strs;
+        for (auto& h : held) {
+            strs.push_back(g_gzLeft ? h.first : NULL);
+            strs.push_back(g_gzFailed ? h.second : NULL);
+        }
+        gzipStrings(w.ctx, strs);
+        for (auto& h : held) {
+            if (h.first) mLeftWriter->input(tid, h.first);
+            if (h.second) mFailedWriter->input(tid, h.second);
+        }
+    }
     return true;
 }
 
@@ -750,16 +816,21 @@ bool SingleEndProcessor::process() {
                 // FPL_DEVICE_EMIT=1: the two output strings are assembled on the device from the chunk it still holds
                 // (fpl_emit_fastq_host: first call builds and reports the sizes, second call copies); the loop below then
                 // only applies the per-read side effects
+                // With FPL_DEVICE_GZIP for every open writer, fpl_emit_fastq_gzip_host compresses both texts before the copy.
+                const bool gzLeft = left && g_gzLeft, gzFailed = failedW && g_gzFailed;
+                const bool gzEmit = deviceEmit && (gzLeft || gzFailed) && (!left || gzLeft) && (!failedW || gzFailed);
+                auto emit = gzEmit ? fpl_emit_fastq_gzip_host : fpl_emit_fastq_host;
+                const char* emitName = gzEmit ? "fpl_emit_fastq_gzip_host" : "fpl_emit_fastq_host";
                 if (deviceEmit && n > 0) {
                     int64_t nOut = 0, nFailed = 0;
-                    int erc = fpl_emit_fastq_host(w.ctx, failedW != NULL, NULL, 0, &nOut, NULL, 0, &nFailed);
-                    if (erc < 0) check(erc, "fpl_emit_fastq_host");
+                    int erc = emit(w.ctx, failedW != NULL, NULL, 0, &nOut, NULL, 0, &nFailed);
+                    if (erc < 0) check(erc, emitName);
                     outstr->resize((size_t)nOut);
                     failedOut->resize((size_t)nFailed);
                     if (nOut + nFailed > 0)
-                        check(fpl_emit_fastq_host(w.ctx, failedW != NULL, nOut ? (uint8_t*)&(*outstr)[0] : NULL, nOut, &nOut,
-                                                  nFailed ? (uint8_t*)&(*failedOut)[0] : NULL, nFailed, &nFailed),
-                              "fpl_emit_fastq_host");
+                        check(emit(w.ctx, failedW != NULL, nOut ? (uint8_t*)&(*outstr)[0] : NULL, nOut, &nOut,
+                                   nFailed ? (uint8_t*)&(*failedOut)[0] : NULL, nFailed, &nFailed),
+                              emitName);
                 } else {
                     outstr->reserve(c->n);
                 }
@@ -775,6 +846,8 @@ bool SingleEndProcessor::process() {
                     const fpl_region* rg = ext.regsOf(i, nregs);
                     scatterRead(v, res[i], sg, rg, nregs, config, failedW != NULL, *outstr, *failedOut, scratch, !deviceEmit);
                 }
+                if ((gzLeft || gzFailed) && !(gzEmit && n > 0))
+                    gzipStrings(w.ctx, {gzLeft ? outstr : NULL, gzFailed ? failedOut : NULL});
                 deliver(outstr, failedOut);
                 freeList.push(c);
             }

@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define FPL_ABI_VERSION 5
+#define FPL_ABI_VERSION 6
 
 /* Filter result codes — identical to src/common.h:43-50 (they index FilterResult::mFilterReadStats[32]). */
 enum {
@@ -294,6 +294,39 @@ int fpl_process_fastq_host(fpl_ctx* ctx, const uint8_t* text, int64_t n_bytes, i
  */
 int fpl_emit_fastq_host(fpl_ctx* ctx, int want_failed, uint8_t* out, int64_t out_cap, int64_t* out_bytes,
                         uint8_t* failed, int64_t failed_cap, int64_t* failed_bytes);
+
+/*
+ * Gzip output — the compression step of Writer::writeInternal / libdeflate_gzip_compress (src/writer.cpp:110-126), which the
+ * reference runs once per buffer flush on the writer thread.  Each piece is cut into segments of FPL_GZIP_SEGMENT bytes (the
+ * last one shorter) and each segment becomes one complete RFC 1952 gzip member (header 1f 8b 08, FLG 0, MTIME 0, XFL 0,
+ * OS 255; one dynamic-Huffman deflate block, or stored blocks when those are not larger; CRC-32; ISIZE).  The members of a
+ * piece follow each other in input order, an empty piece gives 0 bytes, and any concatenation of them is a valid
+ * multi-member gzip stream (zlib, isa-l and gzip read it).  Matches never reach outside their segment.  The bytes are a pure
+ * function of the input.  FPL_GZIP_BOUND(n_bytes, n_pieces) bounds the output of n_bytes in n_pieces pieces.
+ */
+#define FPL_GZIP_SEGMENT 65536
+#define FPL_GZIP_BOUND(n_bytes, n_pieces) \
+    ((int64_t)(n_bytes) + 28 * ((int64_t)(n_bytes) / FPL_GZIP_SEGMENT + (int64_t)(n_pieces)))
+
+/*
+ * Compresses n_pieces pieces held back to back in HOST memory (text; piece_bytes[i] bytes each) on the context's device and
+ * stream: the compressed pieces go to out back to back, their sizes to out_piece_bytes[n_pieces].  Fails (< 0) if
+ * out_cap < FPL_GZIP_BOUND(total bytes, n_pieces).  Synchronous; uses the context's grow-only scratch and leaves the
+ * state of the last fpl_process_fastq_host call alone.  Pieces exist because a writer receives one string per 16-read
+ * pack (WriterThread, src/writerthread.cpp:37-48) and each must stay a whole gzip stream.
+ */
+int fpl_gzip_host(fpl_ctx* ctx, const uint8_t* text, const int64_t* piece_bytes, int32_t n_pieces, uint8_t* out,
+                  int64_t out_cap, int64_t* out_piece_bytes);
+
+/*
+ * fpl_emit_fastq_host with both texts compressed in HBM (two pieces of one fpl_gzip_host-style launch) before the copy, so
+ * only the gzip members cross PCIe: the replacement of Writer::writeInternal's libdeflate_gzip_compress (src/writer.cpp:110-126)
+ * for the raw-text path.  Same precondition and the same two-call protocol: *out_bytes / *failed_bytes are always set; 1 = a
+ * buffer is too small and nothing was copied (the compressed text stays on the device for a second call); < 0 on error.
+ * fpl_emit_fastq_host on the same chunk keeps working and returns the uncompressed text.
+ */
+int fpl_emit_fastq_gzip_host(fpl_ctx* ctx, int want_failed, uint8_t* out, int64_t out_cap, int64_t* out_bytes,
+                             uint8_t* failed, int64_t failed_cap, int64_t* failed_bytes);
 
 /* Output reads / masked regions of the last fpl_process_* call (--mask / --break only; *n = 0 otherwise). */
 int fpl_last_segments(fpl_ctx* ctx, fpl_segment* out, int64_t cap, int64_t* n);
